@@ -29,10 +29,16 @@ One step = one pass of the hot path over the rank's job shard:
 `cpu_baseline` / --impl reference: the oracle (C++ port of the reference's Go path, oracle/oracle.cpp)
            timed on the box's usable host cores (affinity and cgroup quota, cordum_b200/hostinfo.py).
 `parity_check`: untimed; every record of every rank's shard against the oracle, mismatches all-reduced.
+
+--dump-outputs DIR: after the timed steps, the decision records of the last timed step (what a caller of
+           cordum_batch_fetch receives for that batch) are written as DIR/<field>.npy, one array per record field in job
+           order (DIR/<field>.rank<r>.npy per rank at N > 1).  The inputs are seeded, so two builds run with the same
+           arguments can be compared output for output.
 """
 from __future__ import annotations
 
 import argparse
+import atexit
 import ctypes as C
 import json
 import os
@@ -44,16 +50,28 @@ import time
 import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True   # a benchmark run leaves the source tree as it found it (it may be read-only)
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 METRIC = "dispatch decisions/sec (policy-eval+route)"
 UNIT = "decisions/s"
 L2_BYTES = 126 << 20
+DECISION_FIELDS = ("decision", "sched_decision", "flags", "route_status", "reason_code", "rule_idx", "worker_slot")
 
 
 def log(*a):
     print(*a, file=sys.stderr, flush=True)
+
+
+def dump_outputs(out_dir: str, rec: np.ndarray, rank: int, world: int):
+    """One .npy per decision-record field.  The u8 fields are exact in float32; rule_idx and worker_slot (int32) go out
+    as float64 so that no value is rounded.  At 1M jobs: 5 x 4 MB + 2 x 8 MB."""
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = ".rank%d" % rank if world > 1 else ""
+    for f in DECISION_FIELDS:
+        a = rec[f]
+        np.save(os.path.join(out_dir, f + suffix + ".npy"), a.astype(np.float32 if a.dtype.itemsize == 1 else np.float64))
 
 
 def measured_peaks():
@@ -79,6 +97,7 @@ class ClockSampler:
         try:
             self.p = subprocess.Popen(["nvidia-smi", "-i", str(self.device), "--query-gpu=" + self.Q,
                                        "--format=csv,noheader,nounits", "-lms", "50"], stdout=self.f, stderr=subprocess.DEVNULL)
+            atexit.register(self.p.kill)   # no sampler outlives the run: --value-only and failed checks never reach stop()
         except OSError:
             self.p = None
 
@@ -320,6 +339,8 @@ def run_cuda(args, rank: int, world: int, local_rank: int):
     # (same jobs; only the load table changed, so compare policy fields)
     chk = batches[(args.warmup + args.steps - 1) % n_rot].fetch()
     assert np.array_equal(chk["decision"], ref_result["decision"]) and np.array_equal(chk["rule_idx"], ref_result["rule_idx"])
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, chk, rank, world)   # before the parity epoch below overwrites batches[0]'s records
 
     # parity of the sharded path, exchange included: one more epoch with a known delta set, then EVERY rank compares
     # EVERY record of its shard with the oracle evaluated on the table all ranks' slices add up to (checker only,
@@ -352,7 +373,7 @@ def run_cuda(args, rank: int, world: int, local_rank: int):
     oracle_s = time.perf_counter() - t_or
     o.close()
     got = batches[0].fetch()[:n_chk]
-    fields = ("decision", "sched_decision", "flags", "route_status", "reason_code", "rule_idx", "worker_slot")
+    fields = DECISION_FIELDS
     bad_rows = np.zeros(n_chk, dtype=bool)
     for f in fields:
         bad_rows |= got[f] != want[f]
@@ -546,6 +567,8 @@ def main():
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="cordum_b200", choices=["cordum_b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the decision records of the last timed step as DIR/<field>.npy (float32 / float64)")
     ap.add_argument("--value-only", action="store_true", help="diagnostic runs: skip the end-to-end and per-kernel sections")
     ap.add_argument("--parity-sample", type=int, default=0,
                     help="check only the first N jobs of each rank's shard against the oracle (0 = every job; for quick runs)")
@@ -557,6 +580,10 @@ def main():
                          "2-8 GPUs), peer memory over NVLink (CUDA IPC, push kernel inside the ingest graph), or torch.distributed "
                          "all_gather + cordum_workers_set_loads_device")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the CUDA path (the reference leg times a sample sized by its own speed)")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
